@@ -13,6 +13,8 @@ One "step" = one forward+backward sum-product sweep over the whole batch through
   cpu_baseline  fp64 C port of the reference's message schedule (oracle/c) on the host cores
 
 `--impl reference` times that CPU port alone (the reference itself is Julia and cannot run here).
+`--dump-outputs DIR` writes what the timed path returned in its last step as DIR/<name>.npy (see dump_outputs), so that
+two builds can be compared output for output: the inputs are seeded and the same from run to run.
 """
 from __future__ import annotations
 
@@ -33,6 +35,22 @@ D, M, T, BATCH = 4, 4, 1000, 65536
 MSG_PER_STEP = 6                      # rule invocations per (chain, time step), SURVEY.md 8a
 ALGO_BYTES_PER_STEP = 4 * (M + D + D * D)   # 96 B: read y_t, write mu_t and full Sigma_t (SURVEY.md 8d)
 METRIC = "gaussian_messages_per_sec_batched_lgssm_d4_T1000"
+DUMP_BYTES = 64 * 10**6               # --dump-outputs: all files together stay below this
+
+
+def dump_outputs(path, slabs, seed=0):
+    """Writes device outputs as <path>/<name>.npy in their own dtype (float32).  ``slabs`` maps each name to a tensor
+    [G, ..., b] of G * b chains in rank-major slabs (G = 1 on one GPU); the files are [..., chains].  When every chain does
+    not fit in DUMP_BYTES, all arrays keep the same seeded sample of chains, in ascending chain order."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    first = next(iter(slabs.values()))
+    G, b = first.shape[0], first.shape[-1]
+    per_chain = sum(t[0, ..., 0].numel() * t.element_size() for t in slabs.values())
+    k = min(G * b, max(1, (DUMP_BYTES - 4096) // per_chain))           # 4 KB for the .npy headers
+    idx = torch.as_tensor(np.sort(np.random.default_rng(seed).choice(G * b, k, replace=False)), device=first.device)
+    for name, t in slabs.items():
+        np.save(os.path.join(path, name + ".npy"), t[idx // b, ..., idx % b].movedim(0, -1).cpu().numpy())
 
 
 def notebook_model_f32():
@@ -228,6 +246,8 @@ def bench_other_config(args, ctx, dev, emit):
         def step():
             ctx.lgssm(y, **md, smooth=True, out_mean=mean, out_cov=cov, asynchronous=True)
         ms, launches, clocks = timed(step)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"mean": mean[None], "cov": cov[None]})
         for _ in range(3):
             step(); parts.append(ctx.profile_last_ms())
         sweep_ms, gain_ms = float(np.mean([p[0] for p in parts])), float(np.mean([p[1] for p in parts]))
@@ -257,6 +277,8 @@ def bench_other_config(args, ctx, dev, emit):
     yh = (torch.randn(T, batch, device=dev, generator=g).cumsum(0) * 0.5).contiguous()
     outb = torch.empty(T, 4, batch, device=dev)
     ms, launches, clocks = timed(lambda: ctx.hgf_filter(yh, iters=iters, out=outb))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"out": outb[None]})
     msgs = 6 * iters * T * batch
     # end to end: host observations in, host posteriors out through the same entry point
     yhh = torch.empty(T, batch).pin_memory(); yhh.copy_(yh)
@@ -313,7 +335,11 @@ def main():
                     help="BASELINE.json configs[] index: 1 = headline (d=4, batch 65536), 2 = d=64 batch 4096 (tensor-core family), "
                          "3 = HGF T=1000 batch 32768, 20 VMP iterations")
     ap.add_argument("--sweep-variant", type=int, default=0, help="RXG_OPT_SWEEP_VARIANT (0 auto, 1 stash, 2 checkpoint, 3/4 time-segmented)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                    f"(float32; a fixed seeded sample of the chains when all of them exceed {DUMP_BYTES // 10**6} MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path's outputs (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -404,8 +430,12 @@ def main():
     gather = None
     if world == 1:
         ms_per_step, launches = timed(step, args.steps)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"mean": mean[None], "cov": cov[None]})
     else:
         ms_per_step, launches = timed(lambda: step_gather(False), args.steps)          # contract: full gather in the step
+        if args.dump_outputs and rank == 0:                   # the peers wait at the next timed() barrier
+            dump_outputs(args.dump_outputs, {"mean": grp.mean, "cov": grp.cov})
         ms_rep, l_rep = timed(lambda: step_gather(True), args.steps)
         ms_sweep, _ = timed(step, args.steps)
         slab = (mean.numel() + cov.numel()) * 4
